@@ -5,6 +5,7 @@ A "step" is one full KinematicRegistration::ComputeRobotMotion (prior -> converg
 OS1-128-shape synthetic scan (~262 k points) against the 1 M-point voxel map (BASELINE.json configs[3], "cfg4").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload 1..4] [--mode sharded|replicas]
+                    [--dump-outputs DIR]
 
 N > 1 is launched by torchrun, one rank per GPU.  In `sharded` mode (default, the north-star layout) the scan's
 points are split by contiguous index range, the map is replicated, and every IRLS iteration ends with one exchange of
@@ -47,7 +48,27 @@ def parse_args():
     ap.add_argument("--sustained", type=int, default=1000,
                     help="N = 1: registrations of the back-to-back run reported under `sustained` (0 = skip)")
     ap.add_argument("--no-flush", action="store_true", help="diagnostic only: keep L2 warm between steps")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float64), to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+def dump_outputs(d, arrays):
+    """One float64 .npy per returned array; the workloads are seeded, so equal arguments give equal inputs."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
+def result_arrays(res):
+    """The kicp_reg_result of one registration, field by field (per-iteration rows up to `iterations`).  Search windows are handed
+    to warps dynamically, so `sums`, `dx` and `last_dx_norm` of two runs agree to rounding, not bit for bit."""
+    return {"pose": res.pose_np(), "beta": res.beta, "last_dx_norm": res.last_dx_norm, "iterations": res.iterations,
+            "status": res.status, "sums": res.sums_np(), "dx": res.dx_np()}
 
 
 def workload_config(w, extra=None):
@@ -230,7 +251,7 @@ def time_cpu(w, steps, warmup, single_thread_steps=0):
     ts = []
     for _ in range(steps):
         t = time.perf_counter()
-        run()
+        last = run()
         ts.append(time.perf_counter() - t)
     med = statistics.median(ts)
     out = {"value": 1.0 / med, "unit": UNIT, "cores": cores, "kind": kind,
@@ -247,7 +268,7 @@ def time_cpu(w, steps, warmup, single_thread_steps=0):
             run1()
             t1.append(time.perf_counter() - t)
         out["value_1_thread"] = 1.0 / statistics.median(t1)
-    return out, med
+    return out, med, last
 
 
 def run_reference_arm(args):
@@ -258,7 +279,9 @@ def run_reference_arm(args):
     from oracle import workloads as W
     ko.build()
     w = W.Workload(args.workload)
-    cb, sec_per_step = time_cpu(w, args.steps, max(args.warmup, 1), single_thread_steps=1)
+    cb, sec_per_step, last_pose = time_cpu(w, args.steps, max(args.warmup, 1), single_thread_steps=1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"pose": last_pose})
     line = {"metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": 1e3 * sec_per_step, "higher_is_better": True, "scaling": "strong",
             "vs_baseline": None, "dtype": "f64", "data": "synthetic", "impl": "reference",
@@ -472,7 +495,8 @@ def main():
         timing = ctx.last_timing()  # CTA 0 of this rank, last registration: [pass][windows, barrier wait, reduce(+exchange), solve] ns
         jobs = world if (world > 1 and not sharded) else 1  # replicas: every rank finishes its own registrations
         out = {"value": jobs * args.steps / (total_ms * 1e-3), "ms_per_step": total_ms / args.steps, "prof": prof,
-               "launches": launches, "result": results[args.warmup], "n_local": hi - lo, "timing": timing}
+               "launches": launches, "result": results[args.warmup], "last_result": results[-1], "n_local": hi - lo,
+               "timing": timing}
 
         # e2e: host buffers through the public synchronous call, copies inside the timed region
         out_pose = np.empty(7)
@@ -594,9 +618,11 @@ def main():
                       "tolerance": "1e-6 m / 1e-7 rad vs the CPU oracle (sequential-order FP64 restatement); float32 uploads "
                                    "included (the workload's coordinates are float32-representable)"}
         assert pose_delta["translation_m"] <= 1e-6 and pose_delta["rotation_rad"] <= 1e-7, pose_delta
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, result_arrays(main_run["last_result"]))
         cpu_baseline = None
         if world == 1 and not args.no_cpu_baseline:
-            cpu_baseline, _ = time_cpu(w, 5, 1, single_thread_steps=1)
+            cpu_baseline, _, _ = time_cpu(w, 5, 1, single_thread_steps=1)
 
         replay = None
         if world == 1 and args.workload == 4 and not args.no_cpu_baseline and not args.no_replay:

@@ -65,9 +65,33 @@ def pipeline_fixture():
     np.savez_compressed(os.path.join(HERE, "pipeline_seq.npz"), **out)
 
 
+def reference_build_fixture():
+    """The reference's own Registration.cpp on workload cfg2 (1 and 3 threads) and on the scenes of test_golden_cpu.fuzz_cases
+    (one thread), each map filled with the oracle map's voxel-grouped points."""
+    sys.path.insert(0, os.path.dirname(HERE))
+    from test_golden_cpu import fuzz_cases
+    w = W.Workload(2, cache=False)
+    _, _, pts = w.map.export_voxels()
+    rm = ko.RefMap(w.voxel_size, w.max_range, w.max_points_per_voxel)
+    rm.add_points(pts)
+    threads = [1, 3]
+    cfg2 = [rm.register(w.scan, w.last_pose, w.rel_odom, w.tau, threads=t) for t in threads]
+    fuzz, n_map = [], []
+    for om, last, odom, scan, tau, kw in fuzz_cases(ko):
+        _, _, stored = om.export_voxels()
+        rm = ko.RefMap(om.voxel_size, om.max_distance, om.max_points_per_voxel)
+        rm.add_points(stored)
+        n_map.append(rm.num_points())
+        fuzz.append(rm.register(scan, last, odom, tau, threads=1, **kw))
+    np.savez_compressed(os.path.join(HERE, "reference_build.npz"), cfg2_threads=np.array(threads), cfg2_poses=np.array(cfg2),
+                        fuzz_poses=np.array(fuzz), fuzz_map_points=np.array(n_map))
+    print("reference_build cfg2", len(w.scan), "fuzz cases", len(fuzz))
+
+
 if __name__ == "__main__":
     assert ko.ref_available(), "build oracle/_ref first: make -C oracle ref"
     registration_fixture("reg_cfg1", 1)
     registration_fixture("reg_cfg2_small", 2, M=30_000, n_az=450)
     threshold_fixture()
     pipeline_fixture()
+    reference_build_fixture()

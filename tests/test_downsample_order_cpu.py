@@ -10,6 +10,8 @@ import os
 import numpy as np
 import pytest
 
+from oracle.kicp_oracle_py import ref_available
+
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 
 
@@ -70,7 +72,7 @@ def test_downsample_order_modes_keep_the_same_points(oracle, workload):
     assert np.array_equal(ko.voxel_downsample(w.scan, 0.5), base)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/cpp/kinematic_icp"), reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not ref_available(), reason="oracle/_ref not built (the reference's sources were absent at build time)")
 @pytest.mark.parametrize("deskew", [False, True])
 def test_trajectory_sensitivity_to_the_downsample_order(oracle, deskew):
     """The reference's own pipeline sources over the restated KISS-ICP, golden drive, with the down-sample emitting the recalled
